@@ -25,6 +25,11 @@ installed into the git-ignored baseline/_ref/ by scripts/install_reference.py) o
 on the SAME workload: BASELINE configs[1] in full, every step.  Only when baseline/_ref is absent
 does it fall back to the oracle port (bit-exact against the reference, tests/).  `cpu_baseline`
 of the B200 arm is one such step plus BASELINE configs[0] (forward only).
+
+`--steps K` is the number of timed steps of every measurement.  `--dump-outputs DIR` writes what
+the last timed step of the bench workload handed its caller to DIR/<name>.npy (float32; see
+`dump_outputs`).  The inputs depend only on the arguments, so two builds run with the same
+arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -222,6 +227,37 @@ def model_config(wl):
     return {'warm_up': wl['warm_up'], 'dynamic_params': {wl['cls']: wl['dyn']}, 'nmul': NMUL}
 
 
+DUMP_LIMIT = 64 * 10 ** 6     # bytes written by --dump-outputs, .npy headers included
+NPY_HEADER = 128
+
+
+def dump_outputs(dirname, out, loss, grad, shared_grad=None):
+    """Write one training step's results as float32 `dirname/<name>.npy`: every series of `out`
+    (`Model.forward`'s dict), `loss`, `grad_parameters` (the gradient w.r.t. `parameters`) and, if
+    given, `grad_shared` (the all-reduced shared-bias gradient).  When the full arrays exceed
+    DUMP_LIMIT, every per-basin array keeps the same seeded subset of basins, in ascending order."""
+    import numpy as np
+    B = grad.shape[1]
+    arrays = {k: (v, 0 if v.dim() == 1 else 1) for k, v in out.items() if v is not None}
+    arrays.update(loss=(loss, None), grad_parameters=(grad, 1))
+    if shared_grad is not None:
+        arrays['grad_shared'] = (shared_grad, None)
+    for k, (v, ax) in arrays.items():
+        assert ax is None or v.shape[ax] == B, f'{k}: {tuple(v.shape)} has no basin axis of size {B}'
+    room = DUMP_LIMIT - NPY_HEADER * len(arrays) - sum(4 * v.numel() for v, ax in arrays.values() if ax is None)
+    per_basin = sum(4 * v.numel() // B for v, ax in arrays.values() if ax is not None)
+    keep = min(B, room // per_basin)
+    idx = None
+    if keep < B:
+        idx = torch.randperm(B, generator=torch.Generator().manual_seed(SEED))[:keep].sort().values
+    os.makedirs(dirname, exist_ok=True)
+    for k, (v, ax) in arrays.items():
+        v = v.detach()
+        if idx is not None and ax is not None:
+            v = v.index_select(ax, idx.to(v.device))
+        np.save(os.path.join(dirname, k + '.npy'), v.float().cpu().numpy())
+
+
 # algorithmic bytes per basin-timestep (DESIGN.md §4; SURVEY.md §8 d4), nmul = 16:
 # every contract input read once, every output written once
 def bytes_fwd(wl, K=16):
@@ -311,7 +347,9 @@ class CpuArm:
             from oracle import hbv_oracle as O
             out, _ = O.forward_packed(wl['model'], x, pr, nmul=NMUL, warm_up=wl['warm_up'], dynamic_params=wl['dyn'])
         out['streamflow'].sum().backward()
-        return time.perf_counter() - t0
+        dt = time.perf_counter() - t0
+        self.last = (out, pr.grad)
+        return dt
 
     def forward_only(self, x, p):
         """BASELINE configs[0]: forward under no_grad over the run rows only (no warm-up); -> seconds."""
@@ -347,6 +385,9 @@ def run_reference(args):
     tot = 0.0
     for _ in range(args.steps):
         tot += arm.train_step(x, p)
+    if args.dump_outputs:
+        out, grad = arm.last
+        dump_outputs(args.dump_outputs, out, out['streamflow'].sum(), grad)
     val = args.steps * B * wl['T'] / tot
     what = ("unmodified mhpi/hydrodl2 (baseline/_ref): Hbv.forward + autograd" if arm.kind == 'reference'
             else 'oracle port of the reference (oracle/hbv_oracle.py; baseline/_ref absent)')
@@ -573,9 +614,10 @@ def run_b200(args):
                 gstep = GraphedStep(lambda: train_step(model, x_dev, p_dev, allreduce=False), warmup=3, device=dev)
 
                 def step_fn():
-                    _, _, gsh = gstep.replay()
+                    res = gstep.replay()
                     if not NO_ALLREDUCE:
-                        D.allreduce_shared_grad(gsh)
+                        D.allreduce_shared_grad(res[2])
+                    return res
                 graph_note = ('cuda graph replay of the step (hydrodl2_b200.graphs.GraphedStep) + eager NCCL '
                               'all-reduce of the shared gradient')
         except Exception as exc:   # pragma: no cover - depends on driver / NCCL
@@ -583,7 +625,15 @@ def run_b200(args):
             step_fn = lambda: train_step(model, x_dev, p_dev)   # noqa: E731
             step_tail = None
             torch.cuda.synchronize(dev)
-    ms_step = timed(step_fn, args.steps, args.warmup, sampler, tail=step_tail) / args.steps
+    last = []
+    timed_fn = step_fn
+    if args.dump_outputs:
+        def timed_fn():
+            last[:] = [step_fn()]
+    ms_step = timed(timed_fn, args.steps, args.warmup, sampler, tail=step_tail) / args.steps
+    if args.dump_outputs and rank == 0:
+        out, loss, gshared = last[0]
+        dump_outputs(args.dump_outputs, out, loss, p_dev.grad, gshared)
     value = world * B * T_MAIN / (ms_step * 1e-3)
     # The same step with a freshly zeroed dense gradient plane at every step (the clean-plane cache
     # of ops.py switched off): what the 488 MB memset costs.  In the timed loop above the plane of
@@ -629,7 +679,7 @@ def run_b200(args):
             Bs = w2['B']
             model_s, xs, ps = build(w2, Bs, pin=False)
             ps.requires_grad_(True)
-            s_steps, s_warm = 5, 3
+            s_steps, s_warm = args.steps, 3
             ms_s, kms_s = timed_with_kernels(lambda: train_step(model_s, xs, ps), s_steps, s_warm)
             ms_sf, kms_sf = timed_with_kernels(lambda: fwd_only(model_s, xs, ps), s_steps, s_warm)
             ms_s_fill = None          # the same step with the dense plane (re)written at every step
@@ -664,7 +714,7 @@ def run_b200(args):
         spec_.loader.exec_module(cfgs)
         for name, fn, kw in (('c4', cfgs.run_c4, {'B': 2500}), ('c5', cfgs.run_c5, {'B': max(1, 10000 // world)})):
             try:
-                res = fn(3, dev=dev, seed_offset=rank, **kw)
+                res = fn(args.steps, dev=dev, seed_offset=rank, **kw)
             except Exception as exc:      # pragma: no cover - keep the bench line alive
                 at_scale[name] = {'error': f'{type(exc).__name__}: {exc}'}
                 ops.release_grad_planes()      # (idle cached gradient planes of the finished workload)
@@ -775,7 +825,7 @@ def _e2e(args, dev, world, wl, B, model, x_host, p_host, x_dev, p_dev, train_ste
         g_host.copy_(pd.grad, non_blocking=True)
         torch.cuda.current_stream(dev).synchronize()   # the caller needs the results on the host
 
-    e2e_steps = max(3, min(args.steps, 20))
+    e2e_steps = args.steps
     ms_serial = timed(e2e_step, e2e_steps, 3) / e2e_steps
     del xd, pd, g_host, q_host, l_host
 
@@ -856,8 +906,14 @@ def main():
                          'is ~0.55 ms of kernels, about what one eager Python step costs the host, so the '
                          'eager number depends on the host CPU; with several GPUs the all-reduce runs '
                          'eagerly after each replay)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one returned (every output series, the loss, '
+                         'the parameter gradient; rank 0) as DIR/<name>.npy in float32, at most 64 MB in all: '
+                         'beyond that a fixed, seeded subset of basins')
     ap.set_defaults(graph=True)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(3, args.warmup)
     # stdout carries exactly one JSON line: while the run is in progress file descriptor 1 points at
     # stderr (library banners written by native code land there), the line goes to the real stdout

@@ -77,10 +77,8 @@ def long_hourly(dev):
     """BASELINE config 4 at 17,520 steps (tests/test_long_hourly_gpu.py): margins against the fp32
     oracle and the float64 arbiter for every kernel family."""
     import test_long_hourly_gpu as L
-    import numpy as np
     import make_long_hourly as G
-    z = np.load(os.path.join(ROOT, 'tests', 'golden', 'hbv_2_hourly_long.npz'))
-    ref = {k: torch.from_numpy(z[k]) for k in z.files if k != 'meta'}
+    ref = G.load()
     fx = (G, ref) + tuple(G.inputs())
     print('-- hbv_2_hourly, 17,520 hourly steps, fwd + bwd: max-norm relative error vs the fp32 oracle | vs float64 '
           '(oracle fp32 vs float64 in brackets)')
