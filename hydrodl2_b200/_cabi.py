@@ -12,7 +12,7 @@ import os
 
 HBV_MAX_PAR = 20
 HBV_MAX_FLUX = 12
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 VARIANT_HBV, VARIANT_HBV11P, VARIANT_HBV2, VARIANT_HOURLY, VARIANT_ADJ = 0, 1, 2, 3, 4
 SRC_DYN_T, SRC_DYN_LAST, SRC_STA = 0, 1, 2
@@ -66,6 +66,7 @@ class HbvAdjBwdIO(C.Structure):
     _fields_ = [
         ('forcing', _fp), ('dyn', _fp), ('drop', _fp), ('ysol', _fp), ('gqsim', _fp),
         ('gstate_out', _fp), ('gdyn', _fp), ('gstate_in', _fp), ('gdyn_zero_fill', C.c_int32),
+        ('gforcing', _fp),
     ]
 
 

@@ -41,7 +41,11 @@ struct AdjBwdPtrs {
     const float* gqsim; const float* gstate_out;
     float* gdyn; float* gstate_in;
     int zero_fill;
+    float* gforcing;
 };
+// adjoint kernel forms (compile-time): ADJ_GFORCING also produces dL/d(P, T, Ep) into `gforcing`;
+// ADJ_NO_PLANE makes no parameter-gradient stores (gdyn == NULL: forcing / initial-state gradient only)
+constexpr int ADJ_GFORCING = 1, ADJ_NO_PLANE = 2;
 
 // Everything one evaluation of the right-hand side produces.
 struct AdjEval {
@@ -270,12 +274,12 @@ hbv_adj_fwd_kernel(const KDesc d, const AdjFwdPtrs io, const float tol, const in
 }
 
 // One step of the adjoint sweep at the converged end-of-step state y: adds the flux cotangent to
-// gx (= dL/dx_t on entry), solves J^T lambda = gx, returns dL/dp of the step in gp and
-// dL/dx_{t-1} = lambda / dt in gx.
-template <bool BETAET>
+// gx (= dL/dx_t on entry), solves J^T lambda = gx, returns dL/dp of the step in gp,
+// dL/dx_{t-1} = lambda / dt in gx and, with GF, dL/d(P, T, Ep) = lambda^T df/d(P, T, Ep) in gf.
+template <bool BETAET, bool GF>
 __device__ __forceinline__ void adj_bwd_step(const float (&y)[5], const float (&p)[ADJ_NPAR], float P, float T,
                                              float PET, float gQ, float inv_dt, float (&gx)[5],
-                                             float (&gp)[ADJ_NPAR]) {
+                                             float (&gp)[ADJ_NPAR], float (&gf)[3]) {
     AdjEval E;
     adj_eval<BETAET>(y, p, P, T, PET, E);
     AdjJac J;
@@ -318,16 +322,61 @@ __device__ __forceinline__ void adj_bwd_step(const float (&y)[5], const float (&
     gp[HBV_P_UZL] = -c_q01 * p[HBV_P_K0] * E.u;
     gp[HBV_P_K1] = c_q01 * E.SUZ;
     gp[HBV_P_K2] = (gQ - l4) * E.SLZ;
+    if constexpr (GF) {
+        // P: snowfall feeds SNOWPACK; rainfall feeds SM and, through PEFF = (rf + Isnow) sw, SUZ
+        // (the rain/snow mask carries no gradient).  T enters through T - TT only (melt,
+        // refreeze); Ep through et = min(SM, Ep ef).  Q does not depend on the forcings.
+        gf[0] = (T < p[HBV_P_TT]) ? l0 : l2 + c_pe * E.sw;
+        gf[1] = -gp[HBV_P_TT];
+        // (the clamped evaporation factor is recomputed, not kept in AdjEval: one more field there
+        // changes the register allocation of the forward kernel K3)
+        gf[2] = -l2 * (1.f - E.we) * fminf(fmaxf(E.ef1, 0.f), 1.f);
+    }
     // dL/dxt = -lambda^T dG/dxt = lambda / dt
     gx[0] = l0 * inv_dt; gx[1] = l1 * inv_dt; gx[2] = l2 * inv_dt; gx[3] = l3 * inv_dt; gx[4] = l4 * inv_dt;
 
 }
 
-template <bool BETAET, int DM>
-__global__ void __launch_bounds__(128, HBV_ADJ_BWD_MINB)
+// dL/d(P, T, Ep) of step t summed over the nmul components of basin b, stored by the basin's first
+// lane (deterministic, no atomics): butterfly shuffles when the lanes of a basin are an aligned
+// power-of-two group of one warp (`mask`: the warp's lanes), else a sum in component order through
+// the shared-memory slab [NT][3] — the sweep is uniform over the CTA, so its barriers are too.
+__device__ __forceinline__ void adj_store_gforcing(const KDesc& d, float* gforcing, int t, int b, int j, int nmul,
+                                                   bool valid, bool shfl, unsigned mask, float* slab, int tid,
+                                                   float (&g)[3]) {
+    if (shfl) {
+        for (int o = nmul >> 1; o > 0; o >>= 1) {
+            g[0] += __shfl_xor_sync(mask, g[0], o);
+            g[1] += __shfl_xor_sync(mask, g[1], o);
+            g[2] += __shfl_xor_sync(mask, g[2], o);
+        }
+    } else {
+        slab[tid * 3 + 0] = g[0]; slab[tid * 3 + 1] = g[1]; slab[tid * 3 + 2] = g[2];
+        __syncthreads();
+        if (j == 0) {
+            float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+            for (int q = 0; q < nmul; ++q) {
+                a0 += slab[(tid + q) * 3 + 0]; a1 += slab[(tid + q) * 3 + 1]; a2 += slab[(tid + q) * 3 + 2];
+            }
+            g[0] = a0; g[1] = a1; g[2] = a2;
+        }
+        __syncthreads();
+    }
+    if (valid && j == 0) {
+        float* gx = gforcing + ((int64_t)t * d.B + b) * d.nvar;
+        gx[d.i_prcp] = g[0]; gx[d.i_tmean] = g[1]; gx[d.i_pet] = g[2];
+    }
+}
+
+// (the forcing-gradient forms are sized for one CTA per SM fewer: at the 96 registers of
+// HBV_ADJ_BWD_MINB the any-dynamic-set form spills; at 128 none does)
+template <bool BETAET, int DM, int MODE>
+__global__ void __launch_bounds__(128, (MODE & ADJ_GFORCING) ? HBV_ADJ_BWD_MINB - 1 : HBV_ADJ_BWD_MINB)
 hbv_adj_bwd_kernel(const KDesc d, const AdjBwdPtrs io) {
     constexpr int NPAR = ADJ_NPAR;
+    constexpr bool GF = (MODE & ADJ_GFORCING) != 0, PLANE = (MODE & ADJ_NO_PLANE) == 0;
     using DS = DynSet<NPAR, DM>;
+    extern __shared__ __align__(16) float fx_slab[];   // GF, nmul not a power of two: [NT][3]
     const int tid = threadIdx.x, nmul = d.nmul;
     const int bl = tid / nmul, j = tid - bl * nmul;
     const int b_raw = blockIdx.x * d.BPB + bl;
@@ -348,6 +397,8 @@ hbv_adj_bwd_kernel(const KDesc d, const AdjBwdPtrs io) {
     float* gdyn_lane = io.gdyn + (int64_t)b * d.dyn_ncol + j;
     const float inv_nmul = 1.0f / (float)nmul;
     const float inv_dt = d.inv_dt;
+    const bool shfl = (nmul & (nmul - 1)) == 0 && nmul <= 32;     // then NT is a power of two as well
+    const unsigned shfl_mask = blockDim.x >= 32 ? 0xffffffffu : (1u << blockDim.x) - 1u;
 
     float gx[5];
 #pragma unroll
@@ -371,7 +422,7 @@ hbv_adj_bwd_kernel(const KDesc d, const AdjBwdPtrs io) {
         float y[5];
 #pragma unroll
         for (int s = 0; s < 5; ++s) y[s] = ynx[s];
-        if (io.zero_fill) {
+        if (PLANE && io.zero_fill) {
             // fused zero fill (nmul 16): a warp owns two basins, whose gradient rows of step t are
             // one contiguous, 8 B-aligned run; zero it with 8 B stores, then the lanes store their
             // gradients on top.  Row T-1 also receives the static-parameter and routing gradients.
@@ -389,24 +440,32 @@ hbv_adj_bwd_kernel(const KDesc d, const AdjBwdPtrs io) {
         const float gQ = gqn * inv_nmul * d.dt;
         load_all(t - 1);
         apply_dyn<NPAR, DM>(d, dynmask, cur, p, dpd);
-        float gp[NPAR];
-        adj_bwd_step<BETAET>(y, p, cur.P, cur.T, cur.PET, gQ, inv_dt, gx, gp);
+        float gp[NPAR], gf[3];
+        adj_bwd_step<BETAET, GF>(y, p, cur.P, cur.T, cur.PET, gQ, inv_dt, gx, gp, gf);
 
-        float* gr = gdyn_lane + (int64_t)t * dyn_tstride;
+        if constexpr (PLANE) {
+            float* gr = gdyn_lane + (int64_t)t * dyn_tstride;
 #pragma unroll
-        for (int i = 0; i < NPAR; ++i) {
-            if (i < d.n_par) {
-                if (DS::is_dyn(i, dynmask)) { if (valid) gr[d.col[i]] = gp[i] * dpd[i]; }
-                else gacc[i] += gp[i];
+            for (int i = 0; i < NPAR; ++i) {
+                if (i < d.n_par) {
+                    if (DS::is_dyn(i, dynmask)) { if (valid) gr[d.col[i]] = gp[i] * dpd[i]; }
+                    else gacc[i] += gp[i];
+                }
             }
         }
+        // (after the parameter gradient: the reduction's branches must not split the step's
+        // arithmetic from the accumulation above, or its mul-add pairs are no longer fused and
+        // the parameter gradient changes in the last bits)
+        if constexpr (GF) adj_store_gforcing(d, io.gforcing, t, b, j, nmul, valid, shfl, shfl_mask, fx_slab, tid, gf);
     }
-    resolve_params<NPAR, DM>(d, io.dyn, nullptr, io.drop, b, j, p, dpd, &lastmask);
+    if constexpr (PLANE) resolve_params<NPAR, DM>(d, io.dyn, nullptr, io.drop, b, j, p, dpd, &lastmask);
     if (valid) {
-        float* glast = gdyn_lane + (int64_t)(d.T - 1) * dyn_tstride;
+        if constexpr (PLANE) {
+            float* glast = gdyn_lane + (int64_t)(d.T - 1) * dyn_tstride;
 #pragma unroll
-        for (int i = 0; i < NPAR; ++i)
-            if (i < d.n_par && !DS::is_dyn(i, dynmask) && (lastmask & (1u << i))) glast[d.col[i]] = gacc[i] * dpd[i];
+            for (int i = 0; i < NPAR; ++i)
+                if (i < d.n_par && !DS::is_dyn(i, dynmask) && (lastmask & (1u << i))) glast[d.col[i]] = gacc[i] * dpd[i];
+        }
         if (io.gstate_in != nullptr) {
 #pragma unroll
             for (int s = 0; s < 5; ++s) io.gstate_in[s * nlane + lane] = gx[s];
@@ -425,11 +484,14 @@ hbv_adj_bwd_kernel(const KDesc d, const AdjBwdPtrs io) {
 constexpr int ARD = 8;
 constexpr int ASLOT = 8 + 32 * (2 + 5);
 
-template <bool BETAET>
-__global__ void __launch_bounds__(32)
+// (forcing-gradient forms: at least 16 CTAs per SM, i.e. <= 128 registers — left to itself ptxas
+// capped them at 96 registers and spilled)
+template <bool BETAET, int MODE>
+__global__ void __launch_bounds__(32, (MODE & ADJ_GFORCING) ? 16 : 0)
 hbv_adj_bwd_ring_kernel(const KDesc d, const AdjBwdPtrs io) {
     constexpr int NPAR = ADJ_NPAR;
     constexpr int DM = DM_D2;
+    constexpr bool GF = (MODE & ADJ_GFORCING) != 0, PLANE = (MODE & ADJ_NO_PLANE) == 0;
     using DS = DynSet<NPAR, DM>;
     extern __shared__ __align__(16) float ringmem[];
     const int tid = threadIdx.x;
@@ -513,7 +575,7 @@ hbv_adj_bwd_ring_kernel(const KDesc d, const AdjBwdPtrs io) {
         for (int s = 0; s < 5; ++s) y[s] = rp[STB + s * 32 + tid];
         rp += ASLOT;
         if (rp == ring_end) rp = ringmem;
-        if (io.zero_fill) {          // (see the register form)
+        if (PLANE && io.zero_fill) { // (see the register form)
             if (t < d.T - 1 && nbw > 0) {
                 float2* z = reinterpret_cast<float2*>(io.gdyn + ((int64_t)t * d.B + b0w) * d.dyn_ncol);
                 const int n2 = (nbw * d.dyn_ncol) >> 1;
@@ -523,24 +585,30 @@ hbv_adj_bwd_ring_kernel(const KDesc d, const AdjBwdPtrs io) {
         }
         const float gQ = has_gq ? f.w * inv_nmul * d.dt : 0.f;
         apply_dyn<NPAR, DM>(d, dynmask, cur, p, dpd);
-        float gp[NPAR];
-        adj_bwd_step<BETAET>(y, p, cur.P, cur.T, cur.PET, gQ, inv_dt, gx, gp);
-        float* gr = gdyn_lane + (int64_t)t * dyn_tstride;
+        float gp[NPAR], gf[3];
+        adj_bwd_step<BETAET, GF>(y, p, cur.P, cur.T, cur.PET, gQ, inv_dt, gx, gp, gf);
+        if constexpr (PLANE) {
+            float* gr = gdyn_lane + (int64_t)t * dyn_tstride;
 #pragma unroll
-        for (int i = 0; i < NPAR; ++i) {
-            if (i < d.n_par) {
-                if (DS::is_dyn(i, dynmask)) { if (valid) gr[d.col[i]] = gp[i] * dpd[i]; }
-                else gacc[i] += gp[i];
+            for (int i = 0; i < NPAR; ++i) {
+                if (i < d.n_par) {
+                    if (DS::is_dyn(i, dynmask)) { if (valid) gr[d.col[i]] = gp[i] * dpd[i]; }
+                    else gacc[i] += gp[i];
+                }
             }
         }
+        // (a warp is two basins of 16 lanes: two aligned shuffle groups; placed as in the register form)
+        if constexpr (GF) adj_store_gforcing(d, io.gforcing, t, b, j, 16, valid, true, 0xffffffffu, nullptr, tid, gf);
     }
     cp_async_wait<0>();
-    resolve_params<NPAR, DM>(d, io.dyn, nullptr, nullptr, b, j, p, dpd, &lastmask);
+    if constexpr (PLANE) resolve_params<NPAR, DM>(d, io.dyn, nullptr, nullptr, b, j, p, dpd, &lastmask);
     if (valid) {
-        float* glast = gdyn_lane + (int64_t)(d.T - 1) * dyn_tstride;
+        if constexpr (PLANE) {
+            float* glast = gdyn_lane + (int64_t)(d.T - 1) * dyn_tstride;
 #pragma unroll
-        for (int i = 0; i < NPAR; ++i)
-            if (i < d.n_par && !DS::is_dyn(i, dynmask) && (lastmask & (1u << i))) glast[d.col[i]] = gacc[i] * dpd[i];
+            for (int i = 0; i < NPAR; ++i)
+                if (i < d.n_par && !DS::is_dyn(i, dynmask) && (lastmask & (1u << i))) glast[d.col[i]] = gacc[i] * dpd[i];
+        }
         if (io.gstate_in != nullptr) {
 #pragma unroll
             for (int s = 0; s < 5; ++s) io.gstate_in[s * nlane + lane] = gx[s];
@@ -562,15 +630,48 @@ static int launch_adj_fwd(const KDesc& d, const AdjFwdPtrs& io, float tol, int m
     return (int)e;
 }
 
-template <bool BETAET, int DM>
+template <bool BETAET, int DM, int MODE>
 static int launch_adj_bwd(const KDesc& d, const AdjBwdPtrs& io, cudaStream_t st) {
     const int NT = d.BPB * d.nmul;
     const int grid = (d.B + d.BPB - 1) / d.BPB;
-    hbv_adj_bwd_kernel<BETAET, DM><<<grid, NT, 0, st>>>(d, io);
+    const bool pow2 = (d.nmul & (d.nmul - 1)) == 0 && d.nmul <= 32;   // (the kernel's shuffle test)
+    const size_t smem = ((MODE & ADJ_GFORCING) && !pow2) ? (size_t)3 * NT * sizeof(float) : 0;
+    hbv_adj_bwd_kernel<BETAET, DM, MODE><<<grid, NT, smem, st>>>(d, io);
     count_launch();
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) set_error(cudaGetErrorString(e));
     return (int)e;
+}
+
+template <bool BETAET, int DM>
+static int launch_adj_bwd(const KDesc& d, const AdjBwdPtrs& io, int mode, cudaStream_t st) {
+    switch (mode) {
+        case 0: return launch_adj_bwd<BETAET, DM, 0>(d, io, st);
+        case ADJ_GFORCING: return launch_adj_bwd<BETAET, DM, ADJ_GFORCING>(d, io, st);
+        case ADJ_NO_PLANE: return launch_adj_bwd<BETAET, DM, ADJ_NO_PLANE>(d, io, st);
+        default: return launch_adj_bwd<BETAET, DM, ADJ_GFORCING | ADJ_NO_PLANE>(d, io, st);
+    }
+}
+
+template <bool BETAET, int MODE>
+static int launch_adj_bwd_ring(const KDesc& d, const AdjBwdPtrs& io, cudaStream_t st) {
+    const int grid = (d.B + 1) / 2;
+    const size_t smem = (size_t)ARD * ASLOT * sizeof(float);
+    hbv_adj_bwd_ring_kernel<BETAET, MODE><<<grid, 32, smem, st>>>(d, io);
+    count_launch();
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) set_error(cudaGetErrorString(e));
+    return (int)e;
+}
+
+template <bool BETAET>
+static int launch_adj_bwd_ring(const KDesc& d, const AdjBwdPtrs& io, int mode, cudaStream_t st) {
+    switch (mode) {
+        case 0: return launch_adj_bwd_ring<BETAET, 0>(d, io, st);
+        case ADJ_GFORCING: return launch_adj_bwd_ring<BETAET, ADJ_GFORCING>(d, io, st);
+        case ADJ_NO_PLANE: return launch_adj_bwd_ring<BETAET, ADJ_NO_PLANE>(d, io, st);
+        default: return launch_adj_bwd_ring<BETAET, ADJ_GFORCING | ADJ_NO_PLANE>(d, io, st);
+    }
 }
 
 static int adj_prepare(const hbv_desc_t* desc, KDesc& d) {
@@ -609,36 +710,31 @@ int adj_bwd_dispatch(const hbv_desc_t* desc, const hbv_adj_bwd_io_t* io, cudaStr
     KDesc d;
     int rc = adj_prepare(desc, d);
     if (rc) return rc;
-    AdjBwdPtrs p{io->forcing, io->dyn, io->drop, io->ysol, io->gqsim, io->gstate_out, io->gdyn, io->gstate_in, 0};
+    AdjBwdPtrs p{io->forcing, io->dyn, io->drop, io->ysol, io->gqsim, io->gstate_out, io->gdyn, io->gstate_in, 0,
+                 io->gforcing};
     if (io->gdyn_zero_fill) {
-        if (d.nmul != 16 || d.dyn_ncol % 2 != 0 || reinterpret_cast<uintptr_t>(io->gdyn) % 8 != 0) {
+        if (d.nmul != 16 || d.dyn_ncol % 2 != 0 || io->gdyn == nullptr || reinterpret_cast<uintptr_t>(io->gdyn) % 8 != 0) {
             set_error("adj_bwd: gdyn_zero_fill needs nmul 16, an even row width and an 8 B-aligned gdyn");
             return HBV_E_SHAPE;
         }
         p.zero_fill = 1;
     }
+    const int mode = (io->gforcing != nullptr ? ADJ_GFORCING : 0) | (io->gdyn == nullptr ? ADJ_NO_PLANE : 0);
     const int dm = static_dynmask(d, io->drop != nullptr);
     // standard case: the ring form (wide cp.async copies: even rows, 8 / 16 B-aligned bases)
     if (dm == DM_D2 && d.nmul == 16 && d.nvar == 3 && d.i_prcp == 0 && d.i_tmean == 1 && d.i_pet == 2 &&
         d.dyn_ncol % 2 == 0 && d.col[HBV_P_BETA] % 2 == 0 && d.col[HBV_P_BETAET] % 2 == 0 &&
         reinterpret_cast<uintptr_t>(io->dyn) % 8 == 0 && reinterpret_cast<uintptr_t>(io->ysol) % 16 == 0 &&
-        reinterpret_cast<uintptr_t>(io->gdyn) % 8 == 0 && opt(OPT_RING) != 0) {
-        const int grid = (d.B + 1) / 2;
-        const size_t smem = (size_t)ARD * ASLOT * sizeof(float);
-        if (desc->betaet) hbv_adj_bwd_ring_kernel<true><<<grid, 32, smem, st>>>(d, p);
-        else hbv_adj_bwd_ring_kernel<false><<<grid, 32, smem, st>>>(d, p);
-        count_launch();
-        const cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) set_error(cudaGetErrorString(e));
-        return (int)e;
+        reinterpret_cast<uintptr_t>(io->gdyn) % 8 == 0 && opt(OPT_RING) != 0) {   // (gdyn may be NULL)
+        return desc->betaet ? launch_adj_bwd_ring<true>(d, p, mode, st) : launch_adj_bwd_ring<false>(d, p, mode, st);
     }
     if (desc->betaet) {
-        if (dm == 0) return launch_adj_bwd<true, 0>(d, p, st);
-        if (dm == DM_D2) return launch_adj_bwd<true, DM_D2>(d, p, st);
-        return launch_adj_bwd<true, -1>(d, p, st);
+        if (dm == 0) return launch_adj_bwd<true, 0>(d, p, mode, st);
+        if (dm == DM_D2) return launch_adj_bwd<true, DM_D2>(d, p, mode, st);
+        return launch_adj_bwd<true, -1>(d, p, mode, st);
     }
-    if (dm == 0) return launch_adj_bwd<false, 0>(d, p, st);
-    return launch_adj_bwd<false, -1>(d, p, st);
+    if (dm == 0) return launch_adj_bwd<false, 0>(d, p, mode, st);
+    return launch_adj_bwd<false, -1>(d, p, mode, st);
 }
 
 }  // namespace hbv

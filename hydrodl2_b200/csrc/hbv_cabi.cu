@@ -216,7 +216,11 @@ int hbv_b200_adj_fwd(const hbv_desc_t* desc, const hbv_adj_fwd_io_t* io, void* s
 int hbv_b200_adj_bwd(const hbv_desc_t* desc, const hbv_adj_bwd_io_t* io, void* stream) {
     if (!desc || !io) { hbv::set_error("null argument"); return HBV_E_NULL; }
     if (desc->variant != HBV_VARIANT_ADJ) { hbv::set_error("hbv_b200_adj_bwd needs HBV_VARIANT_ADJ"); return HBV_E_VARIANT; }
-    if (!io->forcing || !io->dyn || !io->ysol || !io->gdyn) { hbv::set_error("null input pointer"); return HBV_E_NULL; }
+    if (!io->forcing || !io->dyn || !io->ysol) { hbv::set_error("null input pointer"); return HBV_E_NULL; }
+    if (!io->gdyn) {
+        if (io->gdyn_zero_fill) { hbv::set_error("adj_bwd: gdyn_zero_fill needs gdyn"); return HBV_E_SHAPE; }
+        if (!io->gforcing && !io->gstate_in) { hbv::set_error("adj_bwd: no output (gdyn, gforcing and gstate_in all NULL)"); return HBV_E_NULL; }
+    }
     return hbv::adj_bwd_dispatch(desc, io, (cudaStream_t)stream);
 }
 

@@ -15,6 +15,19 @@ algorithm as written there, restated in ``oracle/hbv_adj_oracle.py``:
   states start at zero (:254), flux read at the end-of-step state (:309-313), nmul mean
   (:315-317), gamma-UH routing with lenF 15 (:319-325).
 
+Extensions (not in the reference; the explicit models have them too):
+
+* gradient w.r.t. the forcings: when ``x_dict['x_phy']`` requires grad, backward fills
+  ``x_phy.grad`` — columns prcp / tmean / pet, warm-up rows included (the warm-up is
+  differentiable here), other columns 0 — from the same adjoint sweep (lambda^T df/d(P, T, Ep)).
+  If ``parameters`` does not require grad (variational precipitation data assimilation), no
+  parameter-gradient tensor is allocated;
+* state carry-over between calls: ``cache_states`` (the next call starts from the last call's
+  final states instead of zeros, its warm-up included), ``get_states()``, ``load_states()``, and
+  ``uh_carry_over`` (with ``cache_states`` and routing: the last lenF - 1 steps of the un-routed
+  flow are routed together with the next call, so a run stepped chunk by chunk gives the routed
+  flow of the one-shot run; inference only).
+
 Deviations (documented in DESIGN.md §4 K3): per-lane stopping rule (the reference's is a
 whole-batch max, :539-544); ``rout_params_name`` typo (:282) fixed; without ``parBETAET`` in
 ``dynamic_params`` the reference indexes a 13th parameter that does not exist (:380-383) — here
@@ -28,7 +41,7 @@ from typing import Any, Optional, Union
 import torch
 
 from ... import _cabi as A
-from ...ops import RunSpec, hbv_adj_run
+from ...ops import RunSpec, hbv_adj_run, route_with_history
 
 
 class HbvAdj(torch.nn.Module):
@@ -53,6 +66,11 @@ class HbvAdj(torch.nn.Module):
         self.nmul = 1
         self.ad_efficient = True
         self.device = device
+        self.cache_states = False
+        self.uh_carry_over = False
+        self._uh_hist = None
+        self.states, self._states_cache = None, None
+        self.state_names = ['SNOWPACK', 'MELTWATER', 'SM', 'SUZ', 'SLZ']
         # Newton controls (extension): reference gtol = 1e-3, <= 4 updates (hbv_adj.py:518-519)
         self.newton_tol = 1e-3
         self.newton_max_updates = 8
@@ -81,11 +99,30 @@ class HbvAdj(torch.nn.Module):
             self.ad_efficient = config.get('ad_efficient', self.ad_efficient)
             self.newton_tol = config.get('newton_tol', self.newton_tol)
             self.newton_max_updates = config.get('newton_max_updates', self.newton_max_updates)
+            self.cache_states = config.get('cache_states', self.cache_states)
+            self.uh_carry_over = config.get('uh_carry_over', self.uh_carry_over)
             if 'parBETAET' in self.dynamic_params:
                 self.parameter_bounds['parBETAET'] = [0.3, 5]
 
         self.set_parameters()
         self.newton_stats = None
+
+    def get_states(self) -> Optional[tuple[torch.Tensor, ...]]:
+        """Final states of the last forward (SNOWPACK, MELTWATER, SM, SUZ, SLZ), each [B, nmul] —
+        a tuple, so that ``load_states(get_states())`` round-trips."""
+        return self._states_cache
+
+    def load_states(self, states: tuple[torch.Tensor, ...]) -> None:
+        """Start the next forward (with ``cache_states``) from `states` (hbv.py:148-168: same
+        checks, same errors; stored detached)."""
+        for state in states:
+            if not isinstance(state, torch.Tensor):
+                raise ValueError("Each element in `states` must be a tensor.")
+        nstates = len(self.state_names)
+        if not (isinstance(states, tuple) and len(states) == nstates):
+            raise ValueError(f"`states` must be a tuple of {nstates} tensors.")
+        self.states = tuple(s.detach().to(self.device, dtype=torch.float32) for s in states)
+        self._uh_hist = None         # a new starting point: no runoff history to route
 
     def set_parameters(self) -> None:
         """hbv_adj.py:99-111."""
@@ -139,12 +176,37 @@ class HbvAdj(torch.nn.Module):
         need = len(self.parameter_bounds) * self.nmul + (2 if self.routing else 0)
         if parameters.shape[-1] < need:
             raise ValueError(f'parameters last dim {parameters.shape[-1]} < {need}')
-        y_init = torch.zeros((5, bs, self.nmul), dtype=torch.float32, device=self.device)   # :254
+        if (not self.states) or (not self.cache_states):
+            y_init = torch.zeros((5, bs, self.nmul), dtype=torch.float32, device=self.device)   # :254
+            self._uh_hist = None
+        else:
+            y_init = torch.stack(tuple(self.states))
+            if tuple(y_init.shape) != (5, bs, self.nmul):
+                raise ValueError(f'cached states have shape {tuple(y_init.shape[1:])}, this call needs '
+                                 f'{(bs, self.nmul)} (basins, nmul)')
+        carry = self.uh_carry_over and self.cache_states and self.routing
+        if carry and torch.is_grad_enabled() and (parameters.requires_grad or x.requires_grad):
+            raise RuntimeError('uh_carry_over is a streaming-inference option: call the model under '
+                               'torch.no_grad() (the routed history of earlier calls carries no gradient)')
         spec_w = self._spec((), routing=False)
-        spec = self._spec(self.dynamic_params, routing=self.routing)
+        spec = self._spec(self.dynamic_params, routing=self.routing and not carry)
         res = hbv_adj_run(spec_w, spec, x, parameters, y_init, drop=self._draw_drop(bs),
                           warm_up=self.warm_up, tol=self.newton_tol,
                           max_updates=self.newton_max_updates)
         self.newton_stats = res['stats']     # int32[2]: max updates, unconverged lane-steps
-        flow = res['routed'] if self.routing else res['qsim']
+        if carry:
+            # route [history of the previous calls ; this run] and keep this run's part
+            n_phy = len(self.parameter_bounds) * self.nmul
+            hist = self._uh_hist
+            if hist is not None and hist.shape[2] != bs:
+                hist = None
+            routed, self._uh_hist = route_with_history(
+                spec, parameters[parameters.shape[0] - 1, :, n_phy:].detach(), parameters.shape[-1],
+                res['qsim'].unsqueeze(0), hist)
+            flow = routed[0]
+        else:
+            flow = res['routed'] if self.routing else res['qsim']
+        self._states_cache = tuple(res['state_out'][i].detach() for i in range(5))
+        if self.cache_states:
+            self.states = self._states_cache
         return {'flow_sim': flow.unsqueeze(-1)}

@@ -749,7 +749,9 @@ class _HbvAdjRun(torch.autograd.Function):
 
     forward : K3 (warm-up rows, all static) -> K3 (run rows) -> K4 (gamma UH, one series)
     backward: K4^T -> K3 adjoint (run) -> K3 adjoint (warm-up); one dense gradient tensor for
-              `parameters`, written in place by the kernels."""
+              `parameters`, written in place by the kernels, and — when `x_phy` requires grad —
+              the forcing gradient of every row, warm-up rows included.  When only `x_phy` needs
+              a gradient, no parameter-gradient plane is allocated at all."""
 
     @staticmethod
     def forward(ctx, spec_w: RunSpec, spec: RunSpec, forcing, dyn, state_in, drop, warm_up, newton, track=True):
@@ -759,7 +761,7 @@ class _HbvAdjRun(torch.autograd.Function):
         nmul, ncol = spec.nmul, dyn.shape[-1]
         T = Tt - warm_up
         tol, maxu = newton
-        need_grad = track and (dyn.requires_grad or state_in.requires_grad)
+        need_grad = track and (dyn.requires_grad or state_in.requires_grad or forcing.requires_grad)
         stream = _stream(dev)
         stats = torch.zeros(2, dtype=torch.int32, device=dev)
 
@@ -820,9 +822,13 @@ class _HbvAdjRun(torch.autograd.Function):
             raise RuntimeError('hydrodl2_b200: backward called but no input required grad')
         # The dense gradient plane: K3's adjoint zeroes the rows it owns itself (gdyn_zero_fill)
         # instead of a 6 GB memset in front of it (BASELINE config 5); what it does not own — the
-        # routing columns of the last row of each call's slice — is cleared here.
+        # routing columns of the last row of each call's slice — is cleared here.  When only the
+        # forcings need a gradient (data assimilation with fixed parameters) there is no plane:
+        # the adjoint gets gdyn = NULL and makes no parameter-gradient stores.
+        need_forcing = ctx.needs_input_grad[2]
+        plane = ctx.needs_input_grad[3] or not need_forcing
         nmul = spec.nmul
-        fused = nmul == 16 and ncol % 2 == 0
+        fused = plane and nmul == 16 and ncol % 2 == 0
         n_phy = spec.n_par * nmul
         kept = None
         if fused and REUSE_GRAD_PLANE and drop is None:
@@ -836,8 +842,11 @@ class _HbvAdjRun(torch.autograd.Function):
             gdyn[Tt - 1, :, n_phy:].zero_()
             if warm_up > 0:
                 gdyn[warm_up - 1, :, n_phy:].zero_()
-        else:
+        elif plane:
             gdyn = torch.zeros_like(dyn)
+        else:
+            gdyn = None
+        gforcing = torch.zeros_like(forcing) if need_forcing else None
 
         def desc_of(sp, nT):
             d = make_desc(sp, nT, B, nvar, ncol, 0)
@@ -848,9 +857,14 @@ class _HbvAdjRun(torch.autograd.Function):
         with torch.cuda.device(dev):
             gq = None if g_q is None else g_q.contiguous()
             if spec.routing and g_rout is not None:
-                route_t = dyn[Tt - 1, :, spec.route_col:]
-                g_route = gdyn[Tt - 1, :, spec.route_col:]
-                rdesc = make_route_desc(spec, T, B, ncol)
+                if gdyn is not None:
+                    route_t = dyn[Tt - 1, :, spec.route_col:]
+                    g_route = gdyn[Tt - 1, :, spec.route_col:]
+                    rdesc = make_route_desc(spec, T, B, ncol)
+                else:       # (the routing-parameter gradient K4^T must write goes to a scratch)
+                    route_t = dyn[Tt - 1, :, spec.route_col:spec.route_col + 2].contiguous()
+                    g_route = torch.empty((B, 2), device=dev, dtype=torch.float32)
+                    rdesc = make_route_desc(spec, T, B, 2)
                 nch = lib.hbv_b200_route_chunks(T, B)
                 ws = torch.empty((min(spec.lenF, T), nch, B), device=dev, dtype=torch.float32)
                 g_in = torch.empty((1, T, B), device=dev, dtype=torch.float32)
@@ -867,8 +881,9 @@ class _HbvAdjRun(torch.autograd.Function):
             io.forcing, io.dyn, io.drop = _ptr(forcing[warm_up:]), _ptr(dyn[warm_up:]), _ptr(drop)
             io.ysol, io.gqsim = _ptr(ysol), _ptr(gq)
             io.gstate_out = None if g_state is None else _ptr(g_state.contiguous())
-            io.gdyn, io.gstate_in = _ptr(gdyn[warm_up:]), _ptr(gmid)
+            io.gdyn, io.gstate_in = _ptr(gdyn[warm_up:] if plane else None), _ptr(gmid)
             io.gdyn_zero_fill = int(fused)
+            io.gforcing = _ptr(gforcing[warm_up:] if need_forcing else None)
             with _timed('hbv_adj_bwd', dev):
                 A.check(lib.hbv_b200_adj_bwd(C.byref(desc_of(spec, T)), C.byref(io), stream), 'adj_bwd')
             gstate_in = gmid
@@ -879,19 +894,21 @@ class _HbvAdjRun(torch.autograd.Function):
                 io.ysol, io.gqsim, io.gstate_out = _ptr(ysol_w), None, _ptr(gmid)
                 io.gdyn, io.gstate_in = _ptr(gdyn), _ptr(gstate_in)
                 io.gdyn_zero_fill = int(fused)
+                io.gforcing = _ptr(gforcing)
                 with _timed('hbv_adj_bwd_warmup', dev):
                     A.check(lib.hbv_b200_adj_bwd(C.byref(desc_of(spec_w, warm_up)), C.byref(io), stream), 'adj_bwd(warm-up)')
         if fused and kept is None and REUSE_GRAD_PLANE and drop is None:
             g_route = route_t = io = None                 # (views of the plane: the cache counts references)
             gdyn = _register_plane(spec, dyn, warm_up, gdyn)
-        return (None, None, None, gdyn, gstate_in if state_in.requires_grad else None, None, None, None, None)
+        return (None, None, gforcing, gdyn, gstate_in if state_in.requires_grad else None, None, None, None, None)
 
 
 def hbv_adj_run(spec_w: RunSpec, spec: RunSpec, forcing, dyn, state_in, drop=None, warm_up: int = 0,
                 tol: float = 1e-3, max_updates: int = 8):
     """Implicit-scheme run.  forcing [T_total, B, nvar], dyn [T_total, B, ncol] raw packed
     parameters, state_in [5, B, nmul].  Rows [:warm_up] are the (differentiable) warm-up with
-    static parameters taken from row warm_up-1 (hbv_adj.py:257-274).
+    static parameters taken from row warm_up-1 (hbv_adj.py:257-274).  `forcing`, `dyn` and
+    `state_in` may each require grad; the forcing gradient covers the warm-up rows too.
     Returns dict(qsim [T,B], routed [T,B] or None, state_out, stats int32[2])."""
     _check_cuda(forcing, 'x_phy')
     _check_cuda(dyn, 'parameters')

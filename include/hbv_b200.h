@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define HBV_B200_ABI_VERSION 4
+#define HBV_B200_ABI_VERSION 5
 
 #if defined(__GNUC__)
 #define HBV_API __attribute__((visibility("default")))
@@ -200,7 +200,8 @@ HBV_API int hbv_b200_bwd(const hbv_desc_t* desc, const hbv_bwd_io_t* io, void* s
  * stopping per lane (||G||_inf <= adj_tol, then one polishing update, <= adj_max_updates).
  * hbv_b200_adj_bwd is the adjoint the reference intends at hbv_adj.py:620-633
  * (lambda = (dG/dx)^-T dL/dx; dL/dp = -lambda^T dG/dp; dL/dxt = -lambda^T dG/dxt) with
- * analytic dG/dp in place of core/calc/fdj.py:46-92.
+ * analytic dG/dp in place of core/calc/fdj.py:46-92.  The same sweep also gives the gradient
+ * w.r.t. the forcings, dL/d(P, T, Ep) = lambda^T df/d(P, T, Ep), and the initial state.
  * desc->variant must be HBV_VARIANT_ADJ, n_par 12 or 13 (betaet), parameters packed
  * (HBV_SRC_DYN_T / HBV_SRC_DYN_LAST), dt = 1.
  */
@@ -224,12 +225,22 @@ typedef struct hbv_adj_bwd_io {
     const float* gqsim;        /* [T, B] or NULL                                */
     const float* gstate_out;   /* [5, B, nmul] or NULL                          */
     float* gdyn;               /* [T, B, dyn_ncol]; zero-initialised by the caller unless
-                                  gdyn_zero_fill is set                          */
+                                  gdyn_zero_fill is set.  NULL: no parameter gradient at all (no
+                                  stores to it; gdyn_zero_fill must then be 0 and at least one of
+                                  gforcing / gstate_in given) — e.g. precipitation data
+                                  assimilation, where only dL/dP is wanted and the dense plane
+                                  would be 6 GB at BASELINE config 5 */
     float* gstate_in;          /* [5, B, nmul] or NULL                          */
     int32_t gdyn_zero_fill;    /* 1 (nmul 16, even dyn_ncol only): the kernel zeroes rows 0 .. T-2 of
                                   gdyn itself before it writes its gradients, so the dense plane needs
                                   no memset (6 GB at BASELINE config 5); of row T-1 it writes the
                                   parameter columns only — the caller owns that row's other columns */
+    float* gforcing;           /* [T, B, nvar] or NULL (ABI 5): gradient w.r.t. the forcings, same
+                                  contract as hbv_bwd_io_t.gforcing — ZERO-INITIALISED by the caller;
+                                  the kernel writes columns i_prcp, i_tmean, i_pet of every row of the
+                                  call, each summed over the nmul components (a fixed-order sum, no
+                                  atomics), and leaves the other columns untouched.  The rain/snow
+                                  mask carries no gradient; T receives it through melt and refreeze */
 } hbv_adj_bwd_io_t;
 
 HBV_API int hbv_b200_adj_fwd(const hbv_desc_t* desc, const hbv_adj_fwd_io_t* io, void* stream);
