@@ -20,8 +20,8 @@ CSRC = os.path.join(HERE, 'csrc')
 LIBDIR = os.path.join(HERE, 'lib')
 LIB = os.path.join(LIBDIR, 'libhbv_b200.so')
 SOURCES = ['hbv_cabi.cu', 'hbv_fwd.cu', 'hbv_bwd.cu', 'uh_route.cu', 'pair_route.cu', 'hbv_adj.cu',
-           'hbv_dense.cu', 'hbv_lean.cu', 'hbv_pipe.cu', 'fill.cu', 'allreduce.cu']
-HEADERS = ['hbv_step.cuh', 'hbv_common.cuh', os.path.join('..', '..', 'include', 'hbv_b200.h')]
+           'hbv_dense.cu', 'hbv_lean.cu', 'hbv_pipe.cu', 'fill.cu', 'allreduce.cu', 'hbv_tlm.cu']
+HEADERS = ['hbv_step.cuh', 'hbv_common.cuh', 'hbv_tlm.cuh', os.path.join('..', '..', 'include', 'hbv_b200.h')]
 # Translation units whose explicit template instantiations are compiled as several objects in
 # parallel (-DHBV_TU_PART=k; the source emits all of them when the macro is absent): the
 # standard-layout and the stage-pipelined kernels are a few hundred instantiations each and would

@@ -12,7 +12,7 @@ import os
 
 HBV_MAX_PAR = 20
 HBV_MAX_FLUX = 12
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 VARIANT_HBV, VARIANT_HBV11P, VARIANT_HBV2, VARIANT_HOURLY, VARIANT_ADJ = 0, 1, 2, 3, 4
 SRC_DYN_T, SRC_DYN_LAST, SRC_STA = 0, 1, 2
@@ -52,6 +52,15 @@ class HbvBwdIO(C.Structure):
         ('muwts', _fp), ('ckpt', _fp), ('gflux', _fp * HBV_MAX_FLUX), ('gstate_out', _fp),
         ('gstate_series', _fp), ('gdyn', _fp), ('gsta', _fp), ('gstate_in', _fp),
         ('gdyn_zero_fill', C.c_int32), ('gdyn_rows_before', C.c_int32), ('gforcing', _fp), ('gmuwts', _fp),
+    ]
+
+
+class HbvTlmIO(C.Structure):
+    _fields_ = [
+        ('forcing', _fp), ('dyn', _fp), ('sta', _fp), ('drop', _fp), ('attrs', _fp),
+        ('muwts', _fp), ('state_in', _fp), ('forcing_t', _fp), ('dyn_t', _fp), ('sta_t', _fp),
+        ('muwts_t', _fp), ('state_in_t', _fp), ('flux_t', _fp * HBV_MAX_FLUX), ('state_out_t', _fp),
+        ('series_t', _fp), ('flux', _fp * HBV_MAX_FLUX), ('state_out', _fp),
     ]
 
 
@@ -97,6 +106,7 @@ EXPORTS = (
     'hbv_b200_pair_route_bwd', 'hbv_b200_adj_fwd', 'hbv_b200_adj_bwd', 'hbv_b200_auto_ckpt',
     'hbv_b200_dense_launches', 'hbv_b200_lean_launches', 'hbv_b200_pipe_launches', 'hbv_b200_workspace_bytes',
     'hbv_b200_set_option', 'hbv_b200_get_option', 'hbv_b200_fill_zero', 'hbv_b200_auto_ckpt_desc', 'hbv_b200_copy_cols', 'hbv_b200_memcpy2d', 'hbv_b200_allreduce_buffer_floats', 'hbv_b200_oneshot_allreduce',
+    'hbv_b200_tlm', 'hbv_b200_route_tlm',
 )
 
 _LIB = None
@@ -151,6 +161,11 @@ def load():
     lib.hbv_b200_fwd.argtypes = [C.POINTER(HbvDesc), C.POINTER(HbvFwdIO), C.c_void_p]
     lib.hbv_b200_bwd.restype = C.c_int
     lib.hbv_b200_bwd.argtypes = [C.POINTER(HbvDesc), C.POINTER(HbvBwdIO), C.c_void_p]
+    lib.hbv_b200_tlm.restype = C.c_int
+    lib.hbv_b200_tlm.argtypes = [C.POINTER(HbvDesc), C.POINTER(HbvTlmIO), C.c_void_p]
+    lib.hbv_b200_route_tlm.restype = C.c_int
+    lib.hbv_b200_route_tlm.argtypes = [C.POINTER(HbvRouteDesc), _fp, _fp, _fp, C.c_int64, _fp, C.c_int64,
+                                       _fp, _fp, _fp, C.c_int64, _fp, _fp, C.c_void_p]
     lib.hbv_b200_adj_fwd.restype = C.c_int
     lib.hbv_b200_adj_fwd.argtypes = [C.POINTER(HbvDesc), C.POINTER(HbvAdjFwdIO), C.c_void_p]
     lib.hbv_b200_adj_bwd.restype = C.c_int

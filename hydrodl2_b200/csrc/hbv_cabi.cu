@@ -56,6 +56,7 @@ int fwd_dispatch(const hbv_desc_t* desc, const hbv_fwd_io_t* io, cudaStream_t st
 int bwd_dispatch(const hbv_desc_t* desc, const hbv_bwd_io_t* io, cudaStream_t st);
 int adj_fwd_dispatch(const hbv_desc_t* desc, const hbv_adj_fwd_io_t* io, cudaStream_t st);
 int adj_bwd_dispatch(const hbv_desc_t* desc, const hbv_adj_bwd_io_t* io, cudaStream_t st);
+int tlm_dispatch(const hbv_desc_t* desc, const hbv_tlm_io_t* io, cudaStream_t st);   // hbv_tlm.cu
 
 static int expected_npar(int variant, int betaet) {
     switch (variant) {
@@ -204,6 +205,16 @@ int hbv_b200_bwd(const hbv_desc_t* desc, const hbv_bwd_io_t* io, void* stream) {
     for (int i = 0; i < desc->n_par && i < HBV_MAX_PAR; ++i)
         if (desc->par_src[i] == HBV_SRC_STA ? (!io->sta || !io->gsta) : (!io->dyn || !io->gdyn)) { hbv::set_error("parameter tensor + gradient required"); return HBV_E_NULL; }
     return hbv::bwd_dispatch(desc, io, (cudaStream_t)stream);
+}
+
+int hbv_b200_tlm(const hbv_desc_t* desc, const hbv_tlm_io_t* io, void* stream) {
+    if (!desc || !io) { hbv::set_error("null argument"); return HBV_E_NULL; }
+    if (desc->variant == HBV_VARIANT_ADJ) { hbv::set_error("hbv_b200_tlm does not serve HBV_VARIANT_ADJ"); return HBV_E_VARIANT; }
+    if (!io->forcing || !io->state_in) { hbv::set_error("null input pointer"); return HBV_E_NULL; }
+    if (desc->variant >= HBV_VARIANT_HBV2 && !io->attrs) { hbv::set_error("attrs (Ac, Elevation) required"); return HBV_E_NULL; }
+    for (int i = 0; i < desc->n_par && i < HBV_MAX_PAR; ++i)
+        if (desc->par_src[i] == HBV_SRC_STA ? !io->sta : !io->dyn) { hbv::set_error("parameter tensor required"); return HBV_E_NULL; }
+    return hbv::tlm_dispatch(desc, io, (cudaStream_t)stream);
 }
 
 int hbv_b200_adj_fwd(const hbv_desc_t* desc, const hbv_adj_fwd_io_t* io, void* stream) {

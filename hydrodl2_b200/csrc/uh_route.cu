@@ -243,6 +243,102 @@ uh_param_bwd_kernel(const RDesc d, const float* __restrict__ route,
     g_route[(int64_t)b * d.route_stride + 1] = gth * db_draw;
 }
 
+// ---- K4t: tangent of the routing ------------------------------------------------------------
+// y_t[s][t] = sum_k uh[k] x_t[s][t-k] + uh_t[k] x[s][t-k], with the tangent of the normalised
+// gamma UH  uh_t[k] = uh[k] ((ln t_k - sum_j uh_j ln t_j) aa_t + (t_k - sum_j uh_j t_j) th_t / th^2)
+// (the closed form uh_param_bwd_kernel transposes).  Same (basin, time chunk) threads and register
+// windows as uh_conv_kernel, one series per grid plane; BFI partial sums of the tangent planes go
+// to bfi_ws_t.
+__global__ void __launch_bounds__(RB)
+uh_conv_tlm_kernel(const RDesc d, const float* __restrict__ route, const float* __restrict__ route_t,
+                   const float* __restrict__ uh, const float* __restrict__ x, int64_t x_stride,
+                   const float* __restrict__ xt, int64_t xt_stride, float* __restrict__ yt, int64_t yt_stride,
+                   float* __restrict__ bfi_ws_t) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    const int c = blockIdx.y;
+    if (b >= d.B) return;
+    const int ts = c * d.tch;
+    const int te = min(d.T, ts + d.tch);
+    float aa, th, da_draw, db_draw;
+    route_ab(d, route, b, aa, th, da_draw, db_draw);
+    float ra_t = 0.f, rb_t = 0.f;
+    if (route_t != nullptr) {
+        ra_t = __ldg(route_t + (int64_t)b * d.route_stride);
+        rb_t = __ldg(route_t + (int64_t)b * d.route_stride + 1);
+    }
+    const float aa_t = da_draw * ra_t;
+    const float th_t = db_draw * rb_t / (th * th);
+    float u[MAXM], ud[MAXM];
+    float mL = 0.f, mT = 0.f;
+#pragma unroll
+    for (int k = 0; k < MAXM; ++k) {
+        u[k] = (k < d.M) ? __ldg(uh + (int64_t)k * d.B + b) : 0.f;
+        const float tk = (float)k + 0.5f;
+        mL += u[k] * logf(tk);
+        mT += u[k] * tk;
+    }
+#pragma unroll
+    for (int k = 0; k < MAXM; ++k) {
+        const float tk = (float)k + 0.5f;
+        ud[k] = u[k] * ((logf(tk) - mL) * aa_t + (tk - mT) * th_t);
+    }
+
+    const int s = blockIdx.z;
+    const float* xs = x + s * x_stride + b;
+    const float* xts = xt + s * xt_stride + b;
+    float* ys = yt + s * yt_stride + b;
+    float win[MAXM - 1 + MAXM], wint[MAXM - 1 + MAXM];
+#pragma unroll
+    for (int i = 0; i < MAXM - 1; ++i) {
+        const int t = ts - (MAXM - 1) + i;
+        win[i] = (t >= 0) ? __ldg(xs + (int64_t)t * d.B) : 0.f;
+        wint[i] = (t >= 0) ? __ldg(xts + (int64_t)t * d.B) : 0.f;
+    }
+    float acc_sum = 0.f;
+    for (int tb = ts; tb < te; tb += MAXM) {
+#pragma unroll
+        for (int i = 0; i < MAXM; ++i) {
+            const int t = tb + i;
+            win[MAXM - 1 + i] = (t < te) ? __ldg(xs + (int64_t)t * d.B) : 0.f;
+            wint[MAXM - 1 + i] = (t < te) ? __ldg(xts + (int64_t)t * d.B) : 0.f;
+        }
+#pragma unroll
+        for (int i = 0; i < MAXM; ++i) {
+            float acc = 0.f;
+#pragma unroll
+            for (int k = 0; k < MAXM; ++k) {
+                acc = fmaf(u[k], wint[MAXM - 1 + i - k], acc);
+                acc = fmaf(ud[k], win[MAXM - 1 + i - k], acc);
+            }
+            const int t = tb + i;
+            if (t < te) { ys[(int64_t)t * d.B] = acc; acc_sum += acc; }
+        }
+#pragma unroll
+        for (int i = 0; i < MAXM - 1; ++i) { win[i] = win[MAXM + i]; wint[i] = wint[MAXM + i]; }
+    }
+    if (bfi_ws_t != nullptr) {
+        if (s == d.bfi_num) bfi_ws_t[((int64_t)0 * d.nchunk + c) * d.B + b] = acc_sum;
+        if (s == d.bfi_den) bfi_ws_t[((int64_t)1 * d.nchunk + c) * d.B + b] = acc_sum;
+    }
+}
+
+// BFI tangent: the primal sums reduced exactly as bfi_kernel does, the tangent sums the same way
+__global__ void bfi_tlm_kernel(const RDesc d, const float* __restrict__ bfi_ws, const float* __restrict__ bfi_ws_t,
+                               float* __restrict__ bfi_t) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= d.B) return;
+    float num = 0.f, den = 0.f, num_t = 0.f, den_t = 0.f;
+#pragma unroll 8
+    for (int c = 0; c < d.nchunk; ++c) {
+        num += __ldg(bfi_ws + ((int64_t)0 * d.nchunk + c) * d.B + b);
+        den += __ldg(bfi_ws + ((int64_t)1 * d.nchunk + c) * d.B + b);
+        num_t += __ldg(bfi_ws_t + ((int64_t)0 * d.nchunk + c) * d.B + b);
+        den_t += __ldg(bfi_ws_t + ((int64_t)1 * d.nchunk + c) * d.B + b);
+    }
+    const float D = den + d.nearzero;
+    bfi_t[b] = 100.f * ((num_t * D - num * den_t) / (D * D));
+}
+
 // threads (= basins) per CTA of the conv kernels: small CTAs for small B so the (basin-block,
 // chunk) grid still covers the SMs
 static int route_block(int B) { return B >= 8192 ? RB : (B >= 2048 ? 64 : 32); }
@@ -325,6 +421,28 @@ extern "C" int hbv_b200_route_bwd(const hbv_route_desc_t* desc, const float* rou
     const int bpb = 128 / MAXM;
     uh_param_bwd_kernel<<<(d.B + bpb - 1) / bpb, 128, 0, st>>>(d, route, uh, ws, g_route);
     count_launch(2);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) set_error(cudaGetErrorString(e));
+    return (int)e;
+}
+
+extern "C" int hbv_b200_route_tlm(const hbv_route_desc_t* desc, const float* route, const float* route_t,
+                                  const float* q_in, int64_t q_stride, const float* q_in_t, int64_t qt_stride,
+                                  const float* uh, const float* bfi_ws, float* q_out_t, int64_t out_stride,
+                                  float* bfi_t, float* bfi_ws_t, void* stream) {
+    RDesc d;
+    int rc = make_rdesc(desc, d);
+    if (rc) return rc;
+    if (!route || !q_in || !q_in_t || !uh || !q_out_t || (bfi_t && (!bfi_ws || !bfi_ws_t))) {
+        set_error("null pointer"); return HBV_E_NULL;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rb = route_block(d.B);
+    dim3 grid((d.B + rb - 1) / rb, d.nchunk, d.nser);
+    uh_conv_tlm_kernel<<<grid, rb, 0, st>>>(d, route, route_t, uh, q_in, q_stride, q_in_t, qt_stride,
+                                            q_out_t, out_stride, bfi_t ? bfi_ws_t : nullptr);
+    count_launch();
+    if (bfi_t) { bfi_tlm_kernel<<<(d.B + 127) / 128, 128, 0, st>>>(d, bfi_ws, bfi_ws_t, bfi_t); count_launch(); }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) set_error(cudaGetErrorString(e));
     return (int)e;

@@ -20,7 +20,8 @@ from typing import Any, Optional, Union
 import torch
 
 from ... import _cabi as A
-from ...ops import RunSpec, hbv_run, hbv_states_only, route_with_history, start_grad_plane
+from ...ops import (RunSpec, hbv_run, hbv_states_only, hbv_states_only_dual, is_dual, refuse_forward_ad,
+                   route_with_history, start_grad_plane)
 from ._seam import PackedSeam
 
 _FLUX_KEYS = (
@@ -237,10 +238,15 @@ class PackedHbv(PackedSeam, torch.nn.Module):
         if warm_up > 0:
             # the dense gradient plane starts zeroing while the warm-up kernel runs
             gplane = start_grad_plane(spec, parameters, warm_up, reusable=(self.dy_drop == 0))
-            with torch.no_grad():
-                spec_w = self._spec(dyn_names=(), routing=False)
-                current = hbv_states_only(spec_w, x[:warm_up], parameters[:warm_up].detach(),
-                                          None, current)
+            spec_w = self._spec(dyn_names=(), routing=False)
+            if is_dual(parameters, x, current):
+                # forward mode: the warm-up carries tangents into the initial states, as the
+                # reference's no_grad warm-up does (hbv.py:327-346)
+                current = hbv_states_only_dual(spec_w, x[:warm_up], parameters[:warm_up], current)
+            else:
+                with torch.no_grad():
+                    current = hbv_states_only(spec_w, x[:warm_up], parameters[:warm_up].detach(),
+                                              None, current)
 
         drop = self._draw_drop(ngrid)
         res = hbv_run(spec, x[warm_up:], parameters, None, current, drop=drop,
@@ -251,6 +257,8 @@ class PackedHbv(PackedSeam, torch.nn.Module):
             if torch.is_grad_enabled() and parameters.requires_grad:
                 raise RuntimeError('uh_carry_over is a streaming-inference option: call the model under '
                                    'torch.no_grad() (the routed history of earlier calls carries no gradient)')
+            refuse_forward_ad('uh_carry_over (the routed history of earlier calls carries no tangent)',
+                              parameters, x, current)
             n_phy = len(self.parameter_bounds) * self.nmul
             q_run = torch.stack([res['flux'][f] for f in _R2F]).detach()
             hist = self._uh_hist
@@ -304,6 +312,7 @@ class PackedHbv(PackedSeam, torch.nn.Module):
         spec.par_lo, spec.par_hi = [0.0] * n, [1.0] * n
         state_in = torch.stack(tuple(states))
         if self.initialize:
+            refuse_forward_ad('the `initialize` run (its states are detached)', dyn, forcing, state_in)
             out = hbv_states_only(spec, forcing.contiguous(), dyn.detach(), None, state_in)
             return tuple(out[i] for i in range(5))
         if spec.routing:

@@ -16,7 +16,7 @@ from typing import Any, Optional
 import torch
 
 from ... import _cabi as A
-from ...ops import RunSpec, hbv_run, hbv_states_only
+from ...ops import RunSpec, hbv_run, hbv_states_only, refuse_forward_ad
 from ._seam import SplitSeam
 
 _BASE_BOUNDS = {
@@ -223,6 +223,8 @@ class SplitHbv(SplitSeam, torch.nn.Module):
         spec = self._spec(routing and not long_uh)
         if self.initialize:
             # hbv_2.py:630-632: only the storages are returned
+            refuse_forward_ad('`initialize=True` (its states are detached; this includes Hbv_2_mts)',
+                              x, dyn, sta, current)
             with torch.no_grad():
                 spec.state_series = False
                 out = hbv_states_only(spec, x, None if dyn is None else dyn.detach().contiguous(),
@@ -234,6 +236,8 @@ class SplitHbv(SplitSeam, torch.nn.Module):
             if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (dyn, sta)):
                 raise RuntimeError('uh_carry_over is a streaming-inference option: call the model under '
                                    'torch.no_grad() (the routed history of earlier calls carries no gradient)')
+            refuse_forward_ad('uh_carry_over (the routed history of earlier calls carries no tangent)',
+                              x, dyn, sta, current)
             from ...ops import route_with_history
             rc = self._route_col()
             q_run = torch.stack([res['flux'][f] for f in (A.F_QSIM, A.F_Q0, A.F_Q1, A.F_Q2)]).detach()
@@ -296,6 +300,7 @@ class SplitHbv(SplitSeam, torch.nn.Module):
         current = torch.stack(tuple(states))
         x = forcing.contiguous()
         if self.initialize:
+            refuse_forward_ad('`initialize=True` (its states are detached)', x, dyn, sta, current)
             with torch.no_grad():
                 spec.state_series = False
                 out = hbv_states_only(spec, x, None if dyn is None else dyn.detach(), sta.detach(),

@@ -89,6 +89,8 @@ class Hbv_2_hourly(SplitHbv):
                 distr = torch.stack([distr[k] for k in self.distr_parameter_bounds.keys()], dim=1)
                 bounds = tuple((0.0, 1.0) for _ in bounds)
             if self.cache_states:   # streaming: keep <= _max_history steps of runoff history
+                from ...ops import refuse_forward_ad
+                refuse_forward_ad('the streaming runoff history of `cache_states` (it is detached)', out['Qs'])
                 self._qs_buffer.append(out['Qs'].detach())
                 if len(self._qs_buffer) > self._max_history:
                     self._qs_buffer.pop(0)

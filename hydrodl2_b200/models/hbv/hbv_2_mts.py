@@ -121,6 +121,10 @@ class Hbv_2_mts(torch.nn.Module):
         return predictions
 
     def forward(self, x_dict, parameters):
+        from ...ops import refuse_forward_ad
+        flat = [t for p in parameters for t in (p if isinstance(p, (tuple, list)) else (p,))]
+        refuse_forward_ad('Hbv_2_mts (its daily warm-up states are detached)',
+                          *flat, *(v for v in x_dict.values() if isinstance(v, torch.Tensor)))
         device = self.device
         n_units = x_dict['areas'].shape[0]
         high = self.high_freq_model

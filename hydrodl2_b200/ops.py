@@ -18,6 +18,7 @@ from dataclasses import dataclass, field
 from typing import Optional, Sequence
 
 import torch
+import torch.autograd.forward_ad as fwAD
 
 from . import _cabi as A
 
@@ -229,6 +230,69 @@ def hbv_states_only(spec: RunSpec, forcing, dyn, sta, state_in, drop=None, attrs
         with _timed('hbv_fwd_warmup', forcing.device):
             A.check(lib.hbv_b200_fwd(C.byref(d), C.byref(io), _stream(forcing.device)), 'fwd(warm-up)')
     return state_out
+
+
+def is_dual(*tensors) -> bool:
+    """True when any of `tensors` carries a forward-mode tangent (torch.autograd.forward_ad)."""
+    for t in tensors:
+        if isinstance(t, torch.Tensor) and fwAD.unpack_dual(t).tangent is not None:
+            return True
+    return False
+
+
+def refuse_forward_ad(what: str, *tensors) -> None:
+    """Raise NotImplementedError when a path that cannot carry tangents gets dual inputs, instead
+    of returning outputs whose tangent silently misses a contribution."""
+    if is_dual(*tensors):
+        raise NotImplementedError(f'hydrodl2_b200: forward-mode AD (torch.autograd.forward_ad) is not '
+                                  f'supported through {what}')
+
+
+class _StatesOnly(torch.autograd.Function):
+    """The warm-up run with forward-mode tangents: forward = hbv_states_only (K1 without flux
+    outputs), jvp = K1t in states-only mode.  The reference runs its warm-up under no_grad without
+    a detach (hbv.py:327-346), and no_grad does not stop forward-mode tangents, so the tangents of
+    the warm-up's forcings, parameters and initial states reach the run's initial states.  No
+    reverse-mode gradient, as before."""
+
+    @staticmethod
+    def forward(ctx, spec, forcing, dyn, state_in):
+        ctx.spec = spec
+        ctx.save_for_forward(forcing, dyn, state_in)
+        return hbv_states_only(spec, forcing, dyn, None, state_in)
+
+    @staticmethod
+    def jvp(ctx, _spec_t, forcing_t, dyn_t, state_in_t):
+        lib = A.load()
+        spec = ctx.spec
+        forcing, dyn, state_in = ctx.saved_tensors
+        T, B, nvar = forcing.shape
+        d = make_desc(spec, T, B, nvar, dyn.shape[-1], 0)
+        d.ckpt_interval = 0
+        cont = (lambda t: None if t is None else t.to(dtype=torch.float32).contiguous())
+        forcing_t, dyn_t, state_in_t = cont(forcing_t), cont(dyn_t), cont(state_in_t)
+        state_out_t = torch.empty_like(state_in)
+        io = A.HbvTlmIO()
+        io.forcing, io.dyn, io.state_in = _ptr(forcing), _ptr(dyn), _ptr(state_in)
+        io.forcing_t, io.dyn_t, io.state_in_t = _ptr(forcing_t), _ptr(dyn_t), _ptr(state_in_t)
+        io.state_out_t = _ptr(state_out_t)
+        with torch.cuda.device(forcing.device):
+            with _timed('hbv_tlm_warmup', forcing.device):
+                A.check(lib.hbv_b200_tlm(C.byref(d), C.byref(io), _stream(forcing.device)), 'tlm(warm-up)')
+        return state_out_t
+
+    @staticmethod
+    def backward(ctx, _g):
+        return None, None, None, None
+
+
+def hbv_states_only_dual(spec: RunSpec, forcing, dyn, state_in):
+    """hbv_states_only for dual inputs (packed models' warm-up under forward-mode AD): the final
+    state stack carries the tangent of the warm-up.  Runs under no_grad (no reverse-mode gradient
+    through the warm-up, as in the plain path)."""
+    _check_cuda(forcing, 'x_phy')
+    with torch.no_grad():
+        return _StatesOnly.apply(spec, forcing.contiguous(), dyn.contiguous(), state_in.contiguous())
 
 
 # ---- clean gradient planes kept between steps ---------------------------------------------------
@@ -533,6 +597,8 @@ class _HbvRun(torch.autograd.Function):
         ctx.muwts_shape = None if muwts is None else tuple(muwts.shape)
         ctx.gbuf, ctx.gev, ctx.gfused = gbuf, gev, gfused
         ctx.save_for_backward(forcing, dyn, sta, drop, attrs, mu, ckpt, flux, uh, bfi_ws, state_in)
+        ctx.save_for_forward(forcing, dyn, sta, state_in, drop, attrs, mu, flux, uh, bfi_ws)
+        ctx.alias_series = alias_series
         ctx.set_materialize_grads(False)
         outs = list(flux.unbind(0)[:spec.nflux])
         n_r = spec.n_routed if spec.routing else 0
@@ -542,6 +608,83 @@ class _HbvRun(torch.autograd.Function):
         outs.append(state_out)
         outs.append(series)     # None unless spec.state_series
         ctx.n_r = n_r
+        return tuple(outs)
+
+    @staticmethod
+    def jvp(ctx, _spec_t, forcing_t, dyn_t, sta_t, state_in_t, _drop_t, attrs_t, muwts_t, *_rest):
+        """Forward mode: K1t (tangent-linear recurrence) + K4t (tangent of the routing and BFI).
+        A tangent that is None is a zero tangent (NULL to the kernels).  Returns a tangent for
+        every output, laid out like the primal outputs (views of one buffer)."""
+        if attrs_t is not None:
+            raise NotImplementedError('hydrodl2_b200: forward-mode AD with respect to the catchment '
+                                      'attributes (Ac, elevation) is not supported; they enter only '
+                                      'through branch conditions and the lateral-flux factor')
+        lib = A.load()
+        spec: RunSpec = ctx.spec
+        forcing, dyn, sta, state_in, drop, attrs, mu, flux, uh, bfi_ws = ctx.saved_tensors
+        T, B, nvar, dyn_ncol, sta_ncol, mu_ts = ctx.dims
+        dev = forcing.device
+        nmul, nf, n_r, t_off = spec.nmul, spec.nflux, ctx.n_r, ctx.t_off
+        cont = (lambda t: None if t is None else t.to(dtype=torch.float32).contiguous())
+        forcing_t, sta_t, state_in_t = cont(forcing_t), cont(sta_t), cont(state_in_t)
+        dyn_t = cont(dyn_t)
+        mu_t = None
+        if mu is not None and muwts_t is not None:
+            mu_t, _ = _prep_muwts(muwts_t, T, B, nmul, dev)
+        d = make_desc(spec, T, B, nvar, dyn_ncol, sta_ncol, mu_ts)
+        d.ckpt_interval = 0
+        flux_t = torch.empty((A.HBV_MAX_FLUX, T, B), device=dev, dtype=torch.float32)
+        state_out_t = torch.empty((5, B, nmul), device=dev, dtype=torch.float32)
+        series_t = (torch.empty((5, T, B, nmul), device=dev, dtype=torch.float32)
+                    if spec.state_series else None)
+        io = A.HbvTlmIO()
+        io.forcing, io.dyn, io.sta = _ptr(forcing), _ptr(dyn[t_off:] if dyn is not None else None), _ptr(sta)
+        io.drop, io.attrs, io.muwts, io.state_in = _ptr(drop), _ptr(attrs), _ptr(mu), _ptr(state_in)
+        io.forcing_t, io.sta_t, io.muwts_t = _ptr(forcing_t), _ptr(sta_t), _ptr(mu_t)
+        io.dyn_t = _ptr(dyn_t[t_off:] if dyn_t is not None else None)
+        io.state_in_t = _ptr(state_in_t)
+        for f in range(nf):
+            io.flux_t[f] = flux_t.data_ptr() + f * T * B * 4
+        io.state_out_t, io.series_t = _ptr(state_out_t), _ptr(series_t)
+        stream = _stream(dev)
+        routed_t = bfi_t = None
+        with torch.cuda.device(dev):
+            with _timed('hbv_tlm', dev):
+                A.check(lib.hbv_b200_tlm(C.byref(d), C.byref(io), stream), 'tlm')
+            if n_r:
+                # the routing parameters' tangent: the same columns the primal reads them from
+                if spec.route_src == 'dyn_last':
+                    route_p = dyn[dyn.shape[0] - 1, :, spec.route_col:]
+                    route_pt = None if dyn_t is None else dyn_t[dyn_t.shape[0] - 1, :, spec.route_col:]
+                    stride = dyn_ncol
+                else:
+                    route_p = sta[:, spec.route_col:]
+                    route_pt = None if sta_t is None else sta_t[:, spec.route_col:]
+                    stride = sta_ncol
+                rdesc = make_route_desc(spec, T, B, stride)
+                nch = lib.hbv_b200_route_chunks(T, B)
+                routed_t = torch.empty((spec.n_routed, T, B), device=dev, dtype=torch.float32)
+                bfi_ws_t = None
+                if spec.bfi:
+                    bfi_t = torch.empty((B,), device=dev, dtype=torch.float32)
+                    bfi_ws_t = torch.empty((2, nch, B), device=dev, dtype=torch.float32)
+                with _timed('route_tlm', dev):
+                    A.check(lib.hbv_b200_route_tlm(
+                        C.byref(rdesc), route_p.data_ptr(), _ptr(route_pt), flux.data_ptr(), T * B,
+                        flux_t.data_ptr(), T * B, uh.data_ptr(), _ptr(bfi_ws), routed_t.data_ptr(), T * B,
+                        _ptr(bfi_t), _ptr(bfi_ws_t), stream), 'route_tlm')
+            if series_t is not None and ctx.alias_series:
+                # the primal series is a view of the [T + 1, 5, B, nmul] state store: same layout here
+                full = torch.empty((T + 1, 5, B, nmul), device=dev, dtype=torch.float32)
+                view = full[1:].permute(1, 0, 2, 3)
+                view.copy_(series_t)
+                series_t = view
+        outs = list(flux_t.unbind(0)[:nf])
+        if n_r:
+            outs += list(routed_t.unbind(0)[:n_r])
+        outs.append(bfi_t)
+        outs.append(state_out_t)
+        outs.append(series_t)
         return tuple(outs)
 
     @staticmethod
@@ -808,6 +951,11 @@ class _HbvAdjRun(torch.autograd.Function):
         ctx.save_for_backward(forcing, dyn, drop, state_in, ysol_w, ysol, qsim, uh)
         ctx.set_materialize_grads(False)
         return qsim, (routed[0] if routed is not None else qsim.new_zeros(())), state_out, stats
+
+    @staticmethod
+    def jvp(ctx, *_tangents):
+        raise NotImplementedError('hydrodl2_b200: forward-mode AD is not supported for HbvAdj (the implicit '
+                                  'scheme); use reverse mode')
 
     @staticmethod
     def backward(ctx, g_q, g_rout, g_state, _g_stats):

@@ -111,6 +111,11 @@ class _PairRoute(torch.autograd.Function):
         return out
 
     @staticmethod
+    def jvp(ctx, *_tangents):
+        raise NotImplementedError('hydrodl2_b200: forward-mode AD is not supported through the distributed '
+                                  'pair routing or the per-unit UH routing with more than 16 taps (K4\')')
+
+    @staticmethod
     def backward(ctx, g_out):
         lib = A.load()
         qs, par, uh = ctx.saved_tensors

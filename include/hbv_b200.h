@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define HBV_B200_ABI_VERSION 5
+#define HBV_B200_ABI_VERSION 6
 
 #if defined(__GNUC__)
 #define HBV_API __attribute__((visibility("default")))
@@ -191,6 +191,56 @@ HBV_API int hbv_b200_fwd(const hbv_desc_t* desc, const hbv_fwd_io_t* io, void* s
 HBV_API int hbv_b200_bwd(const hbv_desc_t* desc, const hbv_bwd_io_t* io, void* stream);
 
 /*
+ * K1t: tangent-linear recurrence (forward-mode derivative of hbv_b200_fwd, ABI 6).
+ *
+ * For a direction (forcing_t, dyn_t, sta_t, muwts_t, state_in_t) in input space, computes the
+ * directional derivative of every output of hbv_b200_fwd: J v for the flux planes, the final
+ * states and the state series.  One launch, the primal recomputed alongside.
+ *
+ * Inputs: the primal inputs exactly as in hbv_fwd_io_t (same descriptor; ckpt_interval is
+ * ignored).  The tangents have the layouts of their primals:
+ *   forcing_t  [T, B, nvar]           columns i_prcp, i_tmean, i_pet are read
+ *   dyn_t      [T, B, dyn_ncol]       tangent of the raw (or [0,1]) dynamic / packed parameters;
+ *                                     static packed parameters and dropped dynamic ones read
+ *                                     row T-1, as the primal does
+ *   sta_t      [B, sta_ncol]
+ *   muwts_t    [T or 1, B, nmul]      same time stride as muwts (desc->muwts_t_stride); ignored
+ *                                     without muwts
+ *   state_in_t [5, B, nmul]
+ * Each tangent input may be NULL: a zero tangent.  Ac / Elevation carry no tangent.
+ * Outputs (each NULL = skipped):
+ *   flux_t[f]   [T, B] tangent of flux plane f (nmul-reduced like flux[f]; with muwts the
+ *               streamflow tangent is sum_j (muwts_t q + muwts q_t))
+ *   state_out_t [5, B, nmul] tangent of the final states
+ *   series_t    [5, T, B, nmul] tangent of the state after every step
+ *   flux[f], state_out: the primal outputs, as hbv_b200_fwd writes them (optional).
+ * With every flux and flux_t pointer NULL the kernel runs in states-only mode (warm-up).
+ * Sub-gradients follow PyTorch: min at a tie takes the mean of both tangents; clamp passes the
+ * tangent on its bounds; a**b at a = 0 gives 0 for both tangents; masks carry no tangent.
+ */
+typedef struct hbv_tlm_io {
+    const float* forcing;
+    const float* dyn;
+    const float* sta;
+    const uint8_t* drop;
+    const float* attrs;
+    const float* muwts;
+    const float* state_in;
+    const float* forcing_t;
+    const float* dyn_t;
+    const float* sta_t;
+    const float* muwts_t;
+    const float* state_in_t;
+    float* flux_t[HBV_MAX_FLUX];
+    float* state_out_t;
+    float* series_t;
+    float* flux[HBV_MAX_FLUX];
+    float* state_out;
+} hbv_tlm_io_t;
+
+HBV_API int hbv_b200_tlm(const hbv_desc_t* desc, const hbv_tlm_io_t* io, void* stream);
+
+/*
  * K3: implicit (backward-Euler) HBV, `HbvAdj` (models/hbv/hbv_adj.py).
  *
  * hbv_b200_adj_fwd replaces the per-step NewtonSolve.apply loop (hbv_adj.py:689-712 calling
@@ -293,6 +343,25 @@ HBV_API int hbv_b200_route_bwd(const hbv_route_desc_t* desc, const float* route,
                        const float* g_out, int64_t g_stride, uint32_t g_out_mask,
                        const float* g_bfi, float* g_in, int64_t gin_stride,
                        float* g_route, float* ws, void* stream);
+
+/*
+ * K4t: tangent of hbv_b200_route_fwd (ABI 6).
+ *   route_t   [B, route_stride] tangent of the raw / [0,1] routing parameters (columns 0, 1) or
+ *             NULL (zero)
+ *   q_in      nser primal input planes [T, B] (plane stride q_stride), as given to route_fwd
+ *   q_in_t    nser tangent input planes [T, B] (plane stride qt_stride)
+ *   uh        [min(lenF, T), B] the UH weights route_fwd wrote
+ *   bfi_ws    [2, nchunk, B] the BFI partial sums route_fwd wrote (required when bfi_t != NULL)
+ *   q_out_t   nser tangent output planes: conv(uh, q_in_t) + conv(uh_t, q_in), where uh_t is the
+ *             tangent of the normalised gamma UH
+ *   bfi_t     [B] or NULL: tangent of the BFI, 100 (num_t D - num den_t) / D^2 with
+ *             D = den + nearzero, all sums in a fixed order (no atomics)
+ *   bfi_ws_t  [2, nchunk, B] workspace when bfi_t != NULL
+ */
+HBV_API int hbv_b200_route_tlm(const hbv_route_desc_t* desc, const float* route, const float* route_t,
+                               const float* q_in, int64_t q_stride, const float* q_in_t, int64_t qt_stride,
+                               const float* uh, const float* bfi_ws, float* q_out_t, int64_t out_stride,
+                               float* bfi_t, float* bfi_ws_t, void* stream);
 
 /*
  * K4': distributed (gage, unit) pair routing (hbv_2_hourly.py:800-897: distr_routing +
