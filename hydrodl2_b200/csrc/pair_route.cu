@@ -42,7 +42,7 @@ __device__ __forceinline__ float gamma_w(float t, float aa, float th) {
 // hbv_2_hourly.py:858-897).  par: [P, 3] in [0, 1] (route_a, route_b, route_tau).
 // CTA = 32 pairs (lanes: coalesced rows of uh / the d/dUH workspace) x PTY tap threads; a thread
 // evaluates taps ty, ty + PTY, ... (powf + expf each: one thread per pair walking all 72 taps was
-// a 40 / 140 us serial chain on 79 warps); the normalisation sum and the adjoint's six moments are
+// a 40 / 140 us serial chain on 79 warps); the normalisation sum and the adjoint's moments are
 // reduced over the tap threads through shared memory in a fixed order.
 constexpr int PKT = PM / PTY;      // taps per thread
 
@@ -329,7 +329,7 @@ pair_duh_kernel(const PDesc d, const float* __restrict__ gsrc, int g_stride, con
 __global__ void __launch_bounds__(PPB * PTY)
 pair_uh_bwd_kernel(const PDesc d, const float* __restrict__ par, const float* __restrict__ ws,
                    float* __restrict__ gpar) {
-    __shared__ float red[PTY][6][PPB];
+    __shared__ float red[PTY][4][PPB];
     const int px = threadIdx.x % PPB, ty = threadIdx.x / PPB;
     const int p = blockIdx.x * PPB + px;
     const bool pv = p < d.P;
@@ -362,36 +362,60 @@ pair_uh_bwd_kernel(const PDesc d, const float* __restrict__ par, const float* __
         f = tau - fl;
     }
     // g_y[k] = dL/d(shifted uh[k]);  g_u[j] = dL/d(normalised w[j]) = (1-f) g_y[j+kk] + f g_y[j+kk+1]
-    float gf = 0.f, mL = 0.f, mT = 0.f, sL = 0.f, sT = 0.f, s0 = 0.f;
+    // (g_y = 0 outside [0, M): a negative lag, given physically, shifts the UH forward)
+    // With u[j] = w[j] / sum(w), L = log t, s0 = sum g_u u, mL = sum u L, mT = sum u t (sum u = 1):
+    //   d/d(aa) = sum_j (g_u[j] - s0) u[j] (L[j] - mL),   d/d(th) = sum_j (g_u[j] - s0) u[j] (t[j] - mT) / th^2
+    // in this centred form, from the moments of a first pass.  g_u has a common part much larger
+    // than its variation over the taps (every tap's d/dUH is a sum over the same inputs); the
+    // expanded form sum g_u u L - s0 mL cancels that part after rounding it, and came out up to
+    // ~10x further from float64 than the reference's own float32 gradient (which centres g_u).
+    float gu[PKT], lt[PKT];
+    float gf = 0.f, mL = 0.f, mT = 0.f, s0 = 0.f;
+#pragma unroll
+    for (int q = 0; q < PKT; ++q) {
+        const int j = ty + PTY * q;
+        gu[q] = lt[q] = 0.f;
+        w[q] *= inv;                               // u[j]
+        if (j < d.M) {
+            const float t = (float)j + 0.5f;
+            const float u = w[q];
+            float gy0 = 0.f, gy1 = 0.f;
+            const int k0 = j + kk, k1 = j + kk + 1;
+            if (k0 >= 0 && k0 < d.M) for (int c = 0; c < d.nchunk; ++c) gy0 += ws[((int64_t)k0 * d.nchunk + c) * d.P + pc];
+            if (d.lag_uh && k1 >= 0 && k1 < d.M) for (int c = 0; c < d.nchunk; ++c) gy1 += ws[((int64_t)k1 * d.nchunk + c) * d.P + pc];
+            gu[q] = d.lag_uh ? ((1.f - f) * gy0 + f * gy1) : gy0;
+            gf += u * (gy1 - gy0);                 // d/df of (1-f) u[k-kk] + f u[k-kk-1]
+            lt[q] = logf(t);
+            mL += u * lt[q]; mT += u * t; s0 += gu[q] * u;
+        }
+    }
+    red[ty][0][px] = gf; red[ty][1][px] = mL; red[ty][2][px] = mT; red[ty][3][px] = s0;
+    __syncthreads();
+    gf = mL = mT = s0 = 0.f;
+#pragma unroll
+    for (int y = 0; y < PTY; ++y) {                // every thread sums in the same order
+        gf += red[y][0][px]; mL += red[y][1][px]; mT += red[y][2][px]; s0 += red[y][3][px];
+    }
+    __syncthreads();
+    float ca = 0.f, cb = 0.f;
 #pragma unroll
     for (int q = 0; q < PKT; ++q) {
         const int j = ty + PTY * q;
         if (j < d.M) {
             const float t = (float)j + 0.5f;
-            const float u = w[q] * inv;
-            float gy0 = 0.f, gy1 = 0.f;
-            const int k0 = j + kk, k1 = j + kk + 1;
-            if (k0 < d.M) for (int c = 0; c < d.nchunk; ++c) gy0 += ws[((int64_t)k0 * d.nchunk + c) * d.P + pc];
-            if (d.lag_uh && k1 < d.M) for (int c = 0; c < d.nchunk; ++c) gy1 += ws[((int64_t)k1 * d.nchunk + c) * d.P + pc];
-            const float gu = d.lag_uh ? ((1.f - f) * gy0 + f * gy1) : gy0;
-            gf += u * (gy1 - gy0);                 // d/df of (1-f) u[k-kk] + f u[k-kk-1]
-            const float L = logf(t);
-            mL += u * L; mT += u * t;
-            sL += gu * u * L; sT += gu * u * t; s0 += gu * u;
+            const float du = (gu[q] - s0) * w[q];
+            ca += du * (lt[q] - mL);
+            cb += du * (t - mT);
         }
     }
-    red[ty][0][px] = gf; red[ty][1][px] = mL; red[ty][2][px] = mT;
-    red[ty][3][px] = sL; red[ty][4][px] = sT; red[ty][5][px] = s0;
+    red[ty][0][px] = ca; red[ty][1][px] = cb;
     __syncthreads();
     if (ty != 0 || !pv) return;
-    gf = mL = mT = sL = sT = s0 = 0.f;
+    ca = cb = 0.f;
 #pragma unroll
-    for (int y = 0; y < PTY; ++y) {
-        gf += red[y][0][px]; mL += red[y][1][px]; mT += red[y][2][px];
-        sL += red[y][3][px]; sT += red[y][4][px]; s0 += red[y][5][px];
-    }
-    const float gaa = sL - s0 * mL;
-    const float gth = (sT - s0 * mT) / (th * th);
+    for (int y = 0; y < PTY; ++y) { ca += red[y][0][px]; cb += red[y][1][px]; }
+    const float gaa = ca;
+    const float gth = cb / (th * th);
     gpar[p * 3 + 0] = (a > 0.f ? gaa : 0.f) * d.a_span;
     gpar[p * 3 + 1] = (b > 0.f ? gth : 0.f) * d.b_span;
     gpar[p * 3 + 2] = d.lag_uh ? gf * d.t_span : 0.f;
